@@ -16,6 +16,8 @@ One "step" = one full pass of the hot path over the workload (all folds x all st
            the kernel, D2H of the samples and the host epilogue (xfade/unfold), wall clock.
 N > 1    : weak scaling -- the mel is lengthened so every rank owns 19 folds; one NCCL
            all-gather of the sample blocks is inside the timed region.
+--dump-outputs DIR : after the timing, what the timed path returned in its last step, as DIR/<name>.npy (see
+           dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -96,6 +98,23 @@ def measured_peaks():
         return dict(tflops=float(d["bf16_tflops"]), tflops_sustained=float(d.get("bf16_tflops_sustained", d["bf16_tflops"])),
                     hbm_gbs=float(d["hbm_gbs"]), src="measured")
     return dict(tflops=1590.0, tflops_sustained=1400.0, hbm_gbs=6650.0, src="fallback")
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict):
+    """Writes every array as out_dir/<name>.npy (float32 stays float32, everything else becomes float64).  When they
+    come to more than 64 MB together, each is replaced by the same share of its entries (flattened, sorted indices
+    drawn from a fixed seed), so two runs with the same arguments store the same entries."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            k = a.size * DUMP_LIMIT_BYTES // total
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, size=k, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -231,6 +250,7 @@ def run_reference_arm(args):
             if i >= args.warmup:
                 times.append(dt)
         assert len(wav) == (frames_for(world) - 1) * HOP
+        outputs = {"wav": np.asarray(wav)}
         kind = "reference"
         how = ("UNMODIFIED reference WaveRNN.generate() (oracle/_ref, " + ("eager torch CUDA operators on this GPU" if on_cuda else "CPU") +
                ", fp32), whole call: upsample network + fold + 12100-step loop + xfade")
@@ -238,9 +258,10 @@ def run_reference_arm(args):
         from oracle import torch_port
         for i in range(args.warmup + args.steps):
             torch.manual_seed(1234)
-            _, dt = torch_port.generate_segments_torch(sd, mels_f, aux_f, steps=sample_steps)
+            samples, dt = torch_port.generate_segments_torch(sd, mels_f, aux_f, steps=sample_steps)
             if i >= args.warmup:
                 times.append(dt)
+        outputs = {"samples": np.asarray(samples)}
         kind = "port"
         how = "torch-operator port of the reference loop (oracle/torch_port.py; bit-identical samples), loop only"
     per_step = float(np.mean(times))
@@ -254,6 +275,8 @@ def run_reference_arm(args):
             "cpu_baseline": {"value": value, "unit": "samples/s", "cores": threads, "kind": kind, "sample": sample},
             "e2e": {"value": value, "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "x_realtime": value / 22050.0}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     emit(line)
 
 
@@ -334,10 +357,11 @@ def run_ours(args):
         barrier()
         ev[0].record(stream)
         for _ in range(args.steps):
-            device_step()
+            samples = device_step()
         ev[1].record(stream)
         barrier()
     engine.check()
+    outputs = {"samples": samples.cpu().numpy()} if args.dump_outputs else {}
     t_dev = ev[0].elapsed_time(ev[1]) / 1e3
     gpu_launches = engine.launch_count - launches0
     clocks = clk.summary()
@@ -359,6 +383,8 @@ def run_ours(args):
         barrier()
         t_e2e = time.perf_counter() - t0
         assert np.isfinite(wav).all()
+        if args.dump_outputs:
+            outputs["wav"] = wav
 
     times = torch.tensor([t_dev, t_e2e], dtype=torch.float64, device=device)
     if world > 1:
@@ -410,6 +436,8 @@ def run_ours(args):
             line["cpu_baseline"] = cpu
         if args.seg_steps or args.skip_e2e:
             line["partial"] = "profiling run (--seg-steps/--skip-e2e): NOT a bench value"
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -464,6 +492,8 @@ def run_cfg4(args, device, rank, world, local):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     t = float(tt.item())
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {f"wav_{i:02d}": w for i, w in enumerate(wavs)})
         units = sum(folds) * S * args.steps
         value = units / t
         peaks = measured_peaks()
@@ -527,7 +557,12 @@ def main():
                     help="PROFILING ONLY: generate just the first N steps of every fold in the device-timed region "
                          "(keeps ncu captures short); the printed line is then marked partial and is not a bench value")
     ap.add_argument("--skip-e2e", action="store_true", help="PROFILING ONLY: skip the end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timing, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(at most 64 MB in all: a fixed, seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -64,6 +64,12 @@ def weight_fingerprint(sd) -> dict:
     return out
 
 
+def sample_index(n, k, seed):
+    """Sorted indices of a fixed, seeded sample of k out of n entries (the stored sample of a fixture too large to keep
+    whole)."""
+    return np.sort(np.random.default_rng(seed).choice(n, size=min(n, k), replace=False))
+
+
 def first_exceed(diff, thr):
     """First step (axis -1) at which any row exceeds thr, or None."""
     bad = (np.abs(diff) > thr)

@@ -10,7 +10,6 @@ import torch
 
 import helpers
 from oracle import wavernn_oracle as O
-from oracle import ref_shim
 
 
 def test_ctor_state_dict_layout():
@@ -46,7 +45,8 @@ def test_fold_and_xfade_helpers_match_oracle():
 
 
 def test_sliced_conditioning_equals_full_upsample():
-    """Per-rank / chunked conditioning (halo slices) == one UpsampleNetwork call (:186)."""
+    """Per-rank / chunked conditioning (halo slices) == one UpsampleNetwork call (:186).  Up to the last bits: torch's
+    CPU convolution sums in an order that depends on the input length and the thread count."""
     m = helpers.make_model(0, "MOL").eval()
     mel = helpers.make_mel(61)
     mp = torch.nn.functional.pad(mel, (2, 2))
@@ -56,9 +56,9 @@ def test_sliced_conditioning_equals_full_upsample():
         cm, ca = m.conditioning(mp, 0, 61)
         sm, sa = m.conditioning(mp, 20, 45)
     np.testing.assert_allclose(cm.numpy(), full_m[0].numpy(), atol=5e-6)
-    np.testing.assert_array_equal(ca.numpy(), full_a[0].numpy())
+    np.testing.assert_allclose(ca.numpy(), full_a[0].numpy(), rtol=0, atol=2e-6)
     np.testing.assert_allclose(sm.numpy(), full_m[0, 20 * 275:45 * 275].numpy(), atol=5e-6)
-    np.testing.assert_array_equal(sa.numpy(), full_a[0, 20 * 275:45 * 275].numpy())
+    np.testing.assert_allclose(sa.numpy(), full_a[0, 20 * 275:45 * 275].numpy(), rtol=0, atol=2e-6)
     sd = helpers.state_numpy(m)
     om, oa = O.upsample_network(sd, mp[0].numpy(), pad=2)
     np.testing.assert_allclose(full_m[0].numpy(), om, atol=5e-6)
@@ -106,16 +106,16 @@ def test_save_load_roundtrip_and_wav(tmp_path):
     np.testing.assert_allclose(decode_mu_law(g["mulaw_in"], 512, False), g["mulaw_out"], rtol=1e-15)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not mounted")
 def test_public_surface_matches_reference_class():
-    ref = ref_shim.load_reference()
+    """Parameter names of the reference WaveRNN's methods (fixture tests/golden/reference_surface.json,
+    generator tests/golden/make_golden_pins.py)."""
+    import json
     import wavernn_b200 as W
+    ref = json.loads((helpers.GOLDEN / "reference_surface.json").read_text())
     for name in ("forward", "generate", "get_gru_cell", "pad_tensor", "fold_with_overlap", "xfade_and_unfold",
                  "get_step", "log", "load", "save", "num_params", "gen_display"):
-        a = inspect.signature(getattr(ref.WaveRNN, name))
-        b = inspect.signature(getattr(W.WaveRNN, name))
-        assert list(a.parameters) == list(b.parameters), name
-    assert list(inspect.signature(ref.WaveRNN.__init__).parameters) == list(inspect.signature(W.WaveRNN.__init__).parameters)
+        assert ref[name] == list(inspect.signature(getattr(W.WaveRNN, name)).parameters), name
+    assert ref["__init__"] == list(inspect.signature(W.WaveRNN.__init__).parameters)
 
 
 def test_upsample_taps_reproduce_the_interpolation_cascade():
